@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py ... --dump-outputs DIR      also writes the last timed step's outputs to DIR/*.npy (see dump_outputs)
 
 Workload (config[1] of BASELINE.json): probagen P=14%, 1 GiB per GPU, Huff0 4X encode + decode on
 32 KB blocks with the reference harness' parameters (maxSymbolValue 255, tableLog 12, slot =
@@ -96,6 +97,7 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-sg", action="store_true", help="skip the separate scatter/decode/gather line at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (float32 / float64)")
     return ap.parse_args()
 
 
@@ -177,6 +179,35 @@ def compare_all_blocks(codec, g_c, g_cs, w_c, w_cs, slot, nb):
             return False, nb, total, "byte %d of block %d differs" % (int(c), c0 + int(r))
         total += int(sizes[c0:c0 + k].sum())
     return True, nb, total, None
+
+
+DUMP_BLOCKS = 128                                  # blocks sampled by --dump-outputs over all ranks (see dump_outputs)
+
+
+def dump_outputs(d, cbuf, cs, out, res, slot, rank=0, world=1):
+    """What the encode and decode calls of the last timed step returned, as .npy files in `d`, so that two builds can be
+    compared output for output: every block's encode return value (csizes) and decode return value (results) as float64
+    (through int64, so an in-band error code 2^64 - k reads -k), and for a fixed, seeded sample of DUMP_BLOCKS // world
+    blocks per rank (sample_blocks) their compressed bytes (the slot up to the block's return value, zeros after it) and
+    decoded bytes as float32.  In all: DUMP_BLOCKS * (slot + 32 KB) * 4 B (34 MB) plus 16 B per block per rank (0.5 MB per
+    GiB per rank), so at most 38 MB up to 8 ranks of 1 GiB.  With several ranks each writes <name>_rank<r>.npy.
+    Takes numpy arrays or CUDA tensors."""
+    import numpy as np
+
+    def host(x):
+        return x.cpu().numpy() if hasattr(x, "cpu") else x
+    nb = len(cs)
+    idx = np.sort(np.random.default_rng(1 + rank).choice(nb, min(nb, DUMP_BLOCKS // world), replace=False))
+    sizes = host(cs).view(np.int64)
+    comp = host(cbuf[:nb * slot].reshape(nb, slot)[idx]).astype(np.float32)
+    used = np.where((sizes[idx] < 0) | (sizes[idx] > slot), 0, sizes[idx])                  # in-band error codes store nothing
+    comp[np.arange(slot)[None, :] >= used[:, None]] = 0
+    dec = host(out[:nb * BLOCK].reshape(nb, BLOCK)[idx]).astype(np.float32)
+    suffix = "" if world == 1 else "_rank%d" % rank
+    os.makedirs(d, exist_ok=True)
+    for name, a in (("csizes", sizes.astype(np.float64)), ("results", host(res).view(np.int64).astype(np.float64)),
+                    ("sample_blocks", idx.astype(np.float64)), ("compressed", comp), ("decoded", dec)):
+        np.save(os.path.join(d, name + suffix + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -299,6 +330,8 @@ def run_reference(a):
     for _ in range(a.steps):
         x, y = cpu_roundtrip(L, kind, wl, data, cbuf, cs, out, res, threads); tc += x; td += y
     wall = time.perf_counter() - t0
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, cbuf, cs, out, res, SLOT)
     val = n * a.steps / (tc + td) / 1e9
     sample = "%d MiB of the workload's generator stream (%d blocks), all %d host threads, %d steps" % (n >> 20, nb, threads, a.steps)
     line = {"impl": "reference", "metric": METRIC, "value": round(val, 3), "unit": "GB/s", "n_gpus": a.gpus, "steps": a.steps, "warmup": a.warmup,
@@ -414,6 +447,8 @@ def run_b200(a):
     wall1 = time.perf_counter()
     if sampler:
         sampler.stop()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, cbuf, cs, out, res, SLOT, rank, world)
     total_ms = t0.elapsed_time(t1)
     enc_ms = sum(ev[i][0].elapsed_time(ev[i][1]) for i in range(a.steps)) / a.steps
     dec_ms = sum(ev[i][1].elapsed_time(ev[i][2]) for i in range(a.steps)) / a.steps

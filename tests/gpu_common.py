@@ -1,11 +1,12 @@
-"""Helpers for the -m gpu suite: CPU-side compression with the checker (compiled reference when it
-travelled with the snapshot, else the oracle port) into the bench.c slot layout."""
+"""Helpers for the -m gpu suite: CPU-side compression with the checker (the reference: inside a test its recorded
+calls, reference_calls.py; elsewhere, as in smoke(), the compiled library where it was built, else the oracle port)
+into the bench.c slot layout."""
 import ctypes as C
 import os
 
 import numpy as np
 
-from helpers import load_port, load_ref, ptr, REF_SO
+from helpers import load_port, load_ref, ptr
 
 BLOCK = 32768
 SLOT = 512 + BLOCK + (BLOCK >> 7) + 4 + 8
@@ -13,9 +14,11 @@ CODEC = {"fse": 0, "huf": 1, "u16": 2}
 
 
 def checker():
-    """(library, is_reference).  Never reads /root/reference at test time: only a prebuilt .so."""
-    if os.path.exists(REF_SO):
-        return load_ref(), True
+    """(library, is_reference): the reference (inside a test its recorded calls, elsewhere the compiled library where
+    oracle/_ref was built), else the oracle port"""
+    ref = load_ref()
+    if ref is not None:
+        return ref, True
     return load_port(), False
 
 

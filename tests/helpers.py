@@ -2,6 +2,7 @@
 and builds the input zoo modelled on the reference fuzzers' buffers
 (programs/fuzzer.c:157-161: noise, P=1%, 15%, 90%, constant)."""
 import ctypes as C
+import hashlib
 import os
 import subprocess
 import numpy as np
@@ -32,7 +33,6 @@ def _sig(fn, res, *args):
 
 
 _port = None
-_ref = None
 
 
 def load_port():
@@ -83,63 +83,66 @@ def load_port():
     return _port
 
 
-def have_ref():
-    return os.path.exists(REF_SO) or os.path.isdir("/root/reference/lib")
+_ref = None
 
 
 def load_ref():
-    """the unmodified reference library compiled by oracle/Makefile (None if it cannot be had)"""
+    """the unmodified reference library.  Inside a test: as recorded for that test (reference_calls.py), replayed from
+    tests/golden/reference_calls.npz, or the compiled library itself while recording.  Elsewhere (tests/golden/make_golden.py,
+    smoke()): the library compiled by oracle/Makefile into oracle/_ref, or None where it was not built."""
     global _ref
-    if _ref is None:
-        if not os.path.exists(REF_SO):
-            if not os.path.isdir("/root/reference/lib"):
-                return None
-            subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "ref"])
-        L = C.CDLL(REF_SO)
-        P = C.POINTER
-        _sig(L.HIST_count, sz, P(u), P(u), vp, sz)
-        _sig(L.FSE_optimalTableLog, u, u, sz, u)
-        _sig(L.HUF_optimalTableLog, u, u, sz, u)
-        _sig(L.FSE_normalizeCount, sz, P(C.c_short), u, P(u), sz, u)
-        _sig(L.FSE_NCountWriteBound, sz, u, u)
-        _sig(L.FSE_writeNCount, sz, vp, sz, P(C.c_short), u, u)
-        _sig(L.FSE_readNCount, sz, P(C.c_short), P(u), P(u), vp, sz)
-        _sig(L.FSE_buildCTable, sz, vp, P(C.c_short), u, u)
-        _sig(L.FSE_buildCTableU16, sz, vp, P(C.c_short), u, u)
-        _sig(L.FSE_buildDTable, sz, vp, P(C.c_short), u, u)
-        _sig(L.FSE_buildDTableU16, sz, vp, P(C.c_short), u, u)
-        _sig(L.FSE_compress_usingCTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.FSE_decompress_usingDTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.FSE_compress2, sz, vp, sz, vp, sz, u, u)
-        _sig(L.FSE_compress, sz, vp, sz, vp, sz)
-        _sig(L.FSE_decompress, sz, vp, sz, vp, sz)
-        _sig(L.FSE_compressBound, sz, sz)
-        _sig(L.FSE_compressU16, sz, vp, sz, vp, sz, u, u)
-        _sig(L.FSE_decompressU16, sz, vp, sz, vp, sz)
-        _sig(L.HUF_buildCTable, sz, vp, P(u), u, u)
-        _sig(L.HUF_writeCTable, sz, vp, sz, vp, u, u)
-        _sig(L.HUF_compress4X_usingCTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.HUF_compress1X_usingCTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.HUF_compress2, sz, vp, sz, vp, sz, u, u)
-        _sig(L.HUF_compress, sz, vp, sz, vp, sz)
-        _sig(L.HUF_readStats, sz, vp, sz, vp, P(C.c_uint32), P(C.c_uint32), vp, sz)
-        _sig(L.HUF_readDTableX1, sz, vp, vp, sz)
-        _sig(L.HUF_readDTableX2, sz, vp, vp, sz)
-        _sig(L.HUF_decompress4X2_usingDTable, sz, vp, sz, vp, sz, vp); _sig(L.HUF_decompress1X2_usingDTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.HUF_readDTableX2, sz, vp, vp, sz)
-        _sig(L.HUF_decompress4X2_usingDTable, sz, vp, sz, vp, sz, vp); _sig(L.HUF_decompress1X2_usingDTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.HUF_decompress4X1_usingDTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.HUF_decompress4X2_usingDTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.HUF_decompress4X_usingDTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.HUF_decompress1X1_usingDTable, sz, vp, sz, vp, sz, vp)
-        _sig(L.HUF_decompress, sz, vp, sz, vp, sz)
-        _sig(L.HUF_decompress4X1, sz, vp, sz, vp, sz)
-        _sig(L.HUF_decompress4X2, sz, vp, sz, vp, sz)
-        _sig(L.HUF_selectDecoder, C.c_uint32, sz, sz)
-        _sig(L.refshim_compress_blocks, C.c_double, C.c_int, vp, sz, sz, vp, sz, vp, u, u, C.c_int)
-        _sig(L.refshim_decompress_blocks, C.c_double, C.c_int, vp, vp, sz, sz, vp, sz, vp, vp, C.c_int)
-        _ref = L
-    return _ref
+    import reference_calls
+    if reference_calls.active():
+        L = reference_calls.current()
+    elif _ref is not None:
+        return _ref
+    elif not os.path.exists(REF_SO):
+        return None
+    else:
+        L = _ref = C.CDLL(REF_SO)
+    P = C.POINTER
+    _sig(L.HIST_count, sz, P(u), P(u), vp, sz)
+    _sig(L.FSE_optimalTableLog, u, u, sz, u)
+    _sig(L.HUF_optimalTableLog, u, u, sz, u)
+    _sig(L.FSE_normalizeCount, sz, P(C.c_short), u, P(u), sz, u)
+    _sig(L.FSE_NCountWriteBound, sz, u, u)
+    _sig(L.FSE_writeNCount, sz, vp, sz, P(C.c_short), u, u)
+    _sig(L.FSE_readNCount, sz, P(C.c_short), P(u), P(u), vp, sz)
+    _sig(L.FSE_buildCTable, sz, vp, P(C.c_short), u, u)
+    _sig(L.FSE_buildCTableU16, sz, vp, P(C.c_short), u, u)
+    _sig(L.FSE_buildDTable, sz, vp, P(C.c_short), u, u)
+    _sig(L.FSE_buildDTableU16, sz, vp, P(C.c_short), u, u)
+    _sig(L.FSE_compress_usingCTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.FSE_decompress_usingDTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.FSE_compress2, sz, vp, sz, vp, sz, u, u)
+    _sig(L.FSE_compress, sz, vp, sz, vp, sz)
+    _sig(L.FSE_decompress, sz, vp, sz, vp, sz)
+    _sig(L.FSE_compressBound, sz, sz)
+    _sig(L.FSE_compressU16, sz, vp, sz, vp, sz, u, u)
+    _sig(L.FSE_decompressU16, sz, vp, sz, vp, sz)
+    _sig(L.HUF_buildCTable, sz, vp, P(u), u, u)
+    _sig(L.HUF_writeCTable, sz, vp, sz, vp, u, u)
+    _sig(L.HUF_compress4X_usingCTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.HUF_compress1X_usingCTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.HUF_compress2, sz, vp, sz, vp, sz, u, u)
+    _sig(L.HUF_compress, sz, vp, sz, vp, sz)
+    _sig(L.HUF_readStats, sz, vp, sz, vp, P(C.c_uint32), P(C.c_uint32), vp, sz)
+    _sig(L.HUF_readDTableX1, sz, vp, vp, sz)
+    _sig(L.HUF_readDTableX2, sz, vp, vp, sz)
+    _sig(L.HUF_decompress4X2_usingDTable, sz, vp, sz, vp, sz, vp); _sig(L.HUF_decompress1X2_usingDTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.HUF_readDTableX2, sz, vp, vp, sz)
+    _sig(L.HUF_decompress4X2_usingDTable, sz, vp, sz, vp, sz, vp); _sig(L.HUF_decompress1X2_usingDTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.HUF_decompress4X1_usingDTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.HUF_decompress4X2_usingDTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.HUF_decompress4X_usingDTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.HUF_decompress1X1_usingDTable, sz, vp, sz, vp, sz, vp)
+    _sig(L.HUF_decompress, sz, vp, sz, vp, sz)
+    _sig(L.HUF_decompress4X1, sz, vp, sz, vp, sz)
+    _sig(L.HUF_decompress4X2, sz, vp, sz, vp, sz)
+    _sig(L.HUF_selectDecoder, C.c_uint32, sz, sz)
+    _sig(L.refshim_compress_blocks, C.c_double, C.c_int, vp, sz, sz, vp, sz, vp, u, u, C.c_int)
+    _sig(L.refshim_decompress_blocks, C.c_double, C.c_int, vp, vp, sz, sz, vp, sz, vp, vp, C.c_int)
+    return L
 
 
 def ptr(a):
@@ -186,6 +189,23 @@ def zoo(rng, n):
         return rng.choice(256, n, p=w / w.sum()).astype(np.uint8)
     v = rng.integers(0, int(rng.integers(2, 40)), n, dtype=np.uint8)      # small flat alphabet
     return v
+
+
+def small_vectors():
+    """the inputs of tests/golden/vectors_small.npz in order, as (codec, bytes): 0 FSE and 1 Huff0 on the same
+    ragged / edge-sized byte buffer from the zoo, then 2 FSE-U16 on 16-bit symbols"""
+    rng = np.random.default_rng(20260922)
+    sizes = [0, 1, 2, 3, 4, 7, 11, 12, 13, 15, 16, 17, 31, 64, 100, 255, 256, 1000, 1001, 1499, 1500, 4096, 8191, 32765, 32766, 32767, 32768, 65536, 131072]
+    for n in sizes + [int(rng.integers(20, 40000)) for _ in range(40)]:
+        d = np.ascontiguousarray(zoo(rng, n))
+        yield 0, d
+        yield 1, d
+    for n in (2, 3, 16, 1000, 16384, 16383, 40000):
+        yield 2, np.ascontiguousarray(gen_u16(n + 50, 240, float(rng.uniform(0.05, 0.8)), int(rng.integers(1, 1 << 30)))[50:]).view(np.uint8)
+
+
+def sha256(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
 def rand_size(rng, hi=128 * 1024):

@@ -3,14 +3,16 @@
 The reference's own command-line tool (`fse`, compiled from the unmodified sources by oracle/Makefile `cli` into
 oracle/_ref/fse_ref) is the checker: a frame written by our tool must be BYTE-IDENTICAL to the one `fse -e` / `fse -h`
 writes for the same input, and each tool must decode the other's output -- the `make check` round trip of
-programs/Makefile:115-131, plus raw / RLE / partial blocks and every block-size id."""
+programs/Makefile:115-131, plus raw / RLE / partial blocks and every block-size id.  What the reference tool wrote and
+decoded is replayed as SHA-256 digests recorded with it (reference_calls.py)."""
+import hashlib
 import os
 import subprocess
 
 import numpy as np
 import pytest
 
-from helpers import probagen
+from helpers import load_ref, probagen
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -21,6 +23,16 @@ REF = os.path.join(ROOT, "oracle", "_ref", "fse_ref")
 def _run(args):
     r = subprocess.run(args, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, (args, r.stdout[-500:], r.stderr[-800:])
+
+
+def _sha(path):
+    return hashlib.sha256(open(path, "rb").read()).hexdigest()
+
+
+def _ref_output(args, out):
+    """digest of the file the reference tool writes to `out` (while recording)"""
+    _run([REF, "-f"] + [str(x) for x in args] + [str(out)])
+    return _sha(out)
 
 
 def _inputs():
@@ -36,19 +48,19 @@ def _inputs():
 
 @pytest.mark.parametrize("flag", ["-e", "-h"])
 def test_frames_are_byte_identical_to_the_reference_tool_and_cross_decode(tmp_path, flag):
-    if not (os.path.exists(OURS) and os.path.exists(REF)):
-        pytest.skip("fse_b200_file / fse_ref not built")
+    if not os.path.exists(OURS):
+        pytest.skip("fse_b200_file not built")
+    ref = load_ref()
     for name, data in _inputs():
         src = tmp_path / (name + ".bin"); data.tofile(src)
         a = tmp_path / (name + ".ours.fse"); b = tmp_path / (name + ".ref.fse")
         _run([OURS, flag, str(src), str(a)])
-        _run([REF, "-f", flag, str(src), str(b)])
-        fa = open(a, "rb").read(); fb = open(b, "rb").read()
-        assert fa == fb, (name, flag, len(fa), len(fb))
+        want = ref.value("%s %s frame" % (name, flag), lambda: _ref_output([flag, src], b))
+        assert _sha(a) == want, (name, flag)
         da = tmp_path / (name + ".ours.out"); db = tmp_path / (name + ".ref.out")
-        _run([OURS, "-d", str(b), str(da)])                        # we decode the reference's frame
-        _run([REF, "-f", "-d", str(a), str(db)])                   # the reference decodes ours
-        assert open(da, "rb").read() == data.tobytes() == open(db, "rb").read(), (name, flag)
+        _run([OURS, "-d", str(a), str(da)])                        # we decode the reference's frame (identical to ours)
+        theirs = ref.value("%s %s decoded" % (name, flag), lambda: _ref_output(["-d", a], db))      # the reference decodes ours
+        assert open(da, "rb").read() == data.tobytes() and theirs == hashlib.sha256(data.tobytes()).hexdigest(), (name, flag)
 
 
 def test_empty_input_round_trips(tmp_path):
@@ -65,15 +77,17 @@ def test_empty_input_round_trips(tmp_path):
 
 
 def test_every_block_size_id_and_corruption_is_detected(tmp_path):
-    if not (os.path.exists(OURS) and os.path.exists(REF)):
-        pytest.skip("fse_b200_file / fse_ref not built")
+    if not os.path.exists(OURS):
+        pytest.skip("fse_b200_file not built")
+    ref = load_ref()
     data = probagen(200000, 0.14)
     src = tmp_path / "in.bin"; data.tofile(src)
     for bid in range(0, 7):
         a = tmp_path / ("b%d.fse" % bid); o = tmp_path / ("b%d.out" % bid)
         _run([OURS, "-h", "-B%d" % bid, str(src), str(a)])
-        _run([REF, "-f", "-d", str(a), str(o)])
-        assert open(o, "rb").read() == data.tobytes()
+        # the frame the reference decoded when this was recorded, and what it decoded it to
+        theirs = ref.value("-B%d frame decoded" % bid, lambda: _sha(a) + " " + _ref_output(["-d", a], o))
+        assert theirs == _sha(a) + " " + hashlib.sha256(data.tobytes()).hexdigest(), bid
         _run([OURS, "-d", str(a), str(o)])
         assert open(o, "rb").read() == data.tobytes()
     frame = bytearray(open(tmp_path / "b5.fse", "rb").read())

@@ -1,14 +1,12 @@
 """Pins the oracle port (oracle/fse_oracle.c) against the compiled reference (oracle/_ref):
 differential tests over the fuzzers' buffer zoo plus the unit cases of programs/fuzzer.c:282-464.
-CPU only.  Skipped (not failed) where the reference library cannot be had."""
+CPU only.  The reference's side is replayed from its recorded calls (reference_calls.py)."""
 import ctypes as C
 import numpy as np
 import pytest
 
-from helpers import (load_port, load_ref, have_ref, ptr, zoo, rand_size, is_error, err_code,
+from helpers import (load_port, load_ref, ptr, zoo, rand_size, is_error, err_code,
                      probagen, gen_u16)
-
-pytestmark = pytest.mark.skipif(not have_ref(), reason="compiled reference (oracle/_ref) unavailable")
 
 U = C.c_uint
 BOUND = lambda n: 512 + n + (n >> 7) + 4 + 8
